@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the volumetric-triangulation hot path (BASELINE.json metric: volumetric samples/sec).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--mode tc|tc1|simt]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--mode tc|tc1|simt] [--dump-outputs DIR]
 
 One "step" = one eval forward of a batch of synthetic multi-view samples (4 views of 3x384x384 -> 17 joints,
 ResNet-152 backbone, 64^3 grid, softmax aggregation: BASELINE config #2, batch 8 per GPU) through the native
@@ -57,7 +57,34 @@ def parse():
     ap.add_argument("--no-config5", action="store_true", help="N = 1 only: skip the extra line for BASELINE config #5 (algebraic model)")
     ap.add_argument("--no-torch-gpu", action="store_true", help="skip the ATen/cuDNN secondary bars (fp32 and TF32) of the native arm")
     ap.add_argument("--no-calibrate", action="store_true", help="keep PyTorch default init (faster start, degenerate signal)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="native arm, one GPU: after the timed steps, write what the last timed forward returned as DIR/<name>.npy "
+                         "(float32; outputs larger than %d elements as DIR/<name>_sample.npy, the fixed seeded sample "
+                         "lt_b200.testing.golden_sample draws). Same arguments -> same weights and inputs, so two builds can be "
+                         "compared output for output" % DUMP_SAMPLE)
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs dumps the native arm's outputs")
+    return args
+
+
+DUMP_SAMPLE = 1 << 21     # elements kept of a larger output: 8 MB of float32, the four large outputs well under 64 MB
+
+
+def dump_outputs(directory, outs):
+    """The (keypoints, features, volumes, vol_confidences, cuboids, coord_volumes, base_points) of one forward -> .npy files."""
+    from lt_b200 import testing
+    os.makedirs(directory, exist_ok=True)
+    names = ("keypoints_3d", "features", "volumes", "vol_confidences", None, "coord_volumes", "base_points")
+    for name, t in zip(names, outs):
+        if name is None or t is None:          # cuboids are host objects built from base_points; no confidences under softmax
+            continue
+        a = t.detach().float().cpu().numpy()
+        if a.size > DUMP_SAMPLE:
+            name, a = name + "_sample", testing.golden_sample(a, DUMP_SAMPLE)
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def peaks():
@@ -132,7 +159,7 @@ def cpu_oracle_rate(args, steps, sd=None, images=None, batch=None):
 def main_reference(args, rank):
     if rank != 0:
         return
-    steps, warmup = max(1, min(args.steps, 2)), 1
+    steps, warmup = args.steps, 1
     rate, dt, threads, _ = cpu_oracle_rate(args, steps)
     line = {
         "impl": "reference", "metric": METRIC, "value": rate, "unit": "samples/s", "n_gpus": args.gpus, "steps": steps,
@@ -140,7 +167,7 @@ def main_reference(args, rank):
         "dtype": "f32", "data": "synthetic",
         "config": {"workload": "Volumetric(softmax) ResNet-%d, %d views %dx%d, %d^3 grid, batch %d per GPU"
                    % (args.layers, args.views, args.image, args.image, args.volume, args.batch),
-                   "note": "CPU arm: %d timed forward(s) of one batch (bounded sample of the same workload), warm-up = one sample" % steps},
+                   "note": "CPU arm: %d timed forward(s) of one batch (--steps), warm-up = one sample" % steps},
         "cpu_baseline": {"value": rate, "unit": "samples/s", "cores": threads, "kind": "port",
                          "sample": "%d timed forward(s) of a %d-sample batch of %d-view inputs, CPU oracle port (torch fp32 + numpy), %d of %d host threads"
                                    % (steps, args.batch, args.views, threads, os.cpu_count())},
@@ -163,7 +190,7 @@ def torch_gpu_rate(args, dev, sd, images_dev, batch, tf32, steps=None):
         model = lt_b200.VolumetricTriangulationNet(cfg, device=dev, backend="torch")
         model.load_state_dict(sd)
         model = model.to(dev).eval()
-        steps = steps or max(2, min(args.steps, 5))
+        steps = steps or args.steps
         with torch.no_grad():
             for _ in range(3):
                 model(images_dev, None, batch)
@@ -193,7 +220,7 @@ def algebraic_rate(args, dev, vol_model, images_dev, batch, flush):
     alg = alg.to(dev).eval()
     proj = torch.as_tensor(np.ascontiguousarray(testing.image_projections(batch), dtype=np.float32)).to(dev)
     B = images_dev.shape[0]
-    steps = max(3, min(args.steps, 10))
+    steps = args.steps
     with torch.no_grad():
         for _ in range(3):
             out = alg(images_dev, proj, batch)
@@ -406,6 +433,8 @@ def main_native(args, rank, world, local_rank):
     from lt_b200 import testing
     if not torch.cuda.is_available():
         raise SystemExit("bench.py --impl native needs a CUDA device (the native path has no CPU fallback)")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs is implemented for one GPU (the view-sharded step returns key points only)")
     torch.cuda.set_device(local_rank)
     dev = torch.device("cuda", local_rank)
     dist = None
@@ -441,8 +470,11 @@ def main_native(args, rank, world, local_rank):
             parallelism = "dp1"
             h2d = images.numel() * 4
 
+            def forward(img):
+                return model(img, None, batch)
+
             def step(img):
-                return model(img, None, batch)[0]
+                return forward(img)[0]
 
             # ---- device-resident arm: CUDA events around graph replays, L2 flushed between iterations ----
             for _ in range(max(args.warmup, 3)):
@@ -456,12 +488,15 @@ def main_native(args, rank, world, local_rank):
                 flush.zero_()
                 e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                 e0.record()
-                step(images_dev)
+                outs = forward(images_dev)
                 e1.record()
                 evs.append((e0, e1))
             barrier()
             dev_ms = sum(a.elapsed_time(b) for a, b in evs)
             clocks = sampler.summary()
+            if args.dump_outputs:
+                # the graph's output buffers still hold the last timed step; the arms below overwrite them
+                dump_outputs(args.dump_outputs, outs)
 
             # ---- end-to-end arm, synchronous: pinned host images -> device, forward, keypoints -> host ----
             for _ in range(2):

@@ -87,6 +87,24 @@ def make_batch(batch_size, n_views, image_size=384, seed=0, camera_cls=Camera, d
     return images.to(device), batch
 
 
+def dataset_items(n_items, n_views, size=8, dtype=np.float64, seed=0, camera_cls=None):
+    """Seeded dataset items (the per-sample dicts a collate_fn receives) with size x (size + 2) images of `dtype`."""
+    rng = np.random.RandomState(seed)
+    cams = make_cameras(n_views, image_size=size)
+    if camera_cls is not None:
+        cams = [camera_cls(c.R, c.t, c.K) for c in cams]
+    items = []
+    for i in range(n_items):
+        if dtype == np.uint8:
+            imgs = [rng.randint(0, 256, size=(size, size + 2, 3)).astype(np.uint8) for _ in range(n_views)]
+        else:
+            imgs = [rng.randn(size, size + 2, 3).astype(dtype) for _ in range(n_views)]
+        items.append({"images": imgs, "detections": [rng.rand(5) for _ in range(n_views)], "cameras": list(cams),
+                      "keypoints_3d": rng.randn(17, 4).astype(np.float32), "indexes": i,
+                      "pred_keypoints_3d": rng.randn(17, 3)})
+    return items
+
+
 @torch.no_grad()
 def randomize_weights(model, seed=0, calib_size=64, calib_views=2, feat_gain=4.0, branch_gain=0.2):
     """Seeded, non-degenerate weights (SURVEY.md hard part H1).
@@ -205,3 +223,19 @@ def randomize_backbone_weights(model, seed=0, calib_size=128, calib_images=4, br
 
 
 BN_MOMENTUM = 0.1
+
+
+def golden_sample(a, k=2048, seed=0):
+    """A fixed, seeded sample of at most k elements of `a` (all of them when it is no larger), flattened and in index order:
+    stored golden data and dumped benchmark outputs shrink large arrays this way, so both sides draw the same indices."""
+    a = np.asarray(a).reshape(-1)
+    if a.size <= k:
+        return a.copy()
+    return a[np.unique(np.random.RandomState(seed).randint(0, a.size, size=k))]
+
+
+def array_digest(a):
+    """sha256 of an array's dtype, shape and bytes: stored instead of arrays that a test compares for exact equality."""
+    import hashlib
+    a = np.ascontiguousarray(a)
+    return hashlib.sha256(("%s%s" % (a.dtype.str, a.shape)).encode() + a.tobytes()).hexdigest()

@@ -7,7 +7,6 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-REFERENCE = "/root/reference"
 
 
 def pytest_configure(config):
@@ -23,10 +22,6 @@ def pytest_collection_modifyitems(config, items):
     for item in items:
         if "gpu" in item.keywords:
             item.add_marker(skip)
-
-
-def has_reference():
-    return os.path.isdir(os.path.join(REFERENCE, "mvn"))
 
 
 @pytest.fixture(scope="session")

@@ -1,10 +1,11 @@
 """Generate the golden fixtures in this directory from the UNMODIFIED reference.
 
-Run in the authoring container only (needs /root/reference; the GPU box does not have it):
-    python tests/golden/make_golden.py
-It imports karfly/learnable-triangulation-pytorch read-only, feeds it seeded synthetic inputs and the
+Needs a checkout of karfly/learnable-triangulation-pytorch (the tests themselves never do):
+    python tests/golden/make_golden.py <reference checkout> [fixture ...]
+It imports the reference read-only, feeds it seeded synthetic inputs and the
 seeded weight recipe of lt_b200.testing (loaded with strict=True -- which also proves state_dict
 compatibility), and stores small input/output vectors as .npz.  Nothing is copied from the reference.
+With fixture names (e.g. `oracle_vs_reference collate`) only those files are regenerated.
 """
 import os
 import sys
@@ -15,7 +16,9 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-sys.path.insert(0, "/root/reference")
+if len(sys.argv) < 2 or not os.path.isdir(os.path.join(sys.argv[1], "mvn")):
+    raise SystemExit("usage: python tests/golden/make_golden.py <reference checkout> [fixture ...]")
+sys.path.insert(0, os.path.abspath(sys.argv[1]))
 
 import lt_b200  # noqa: E402
 from lt_b200 import testing  # noqa: E402
@@ -134,11 +137,112 @@ def gen_state_dict_keys():
         json.dump({k: list(v.shape) for k, v in ref.state_dict().items()}, f)
 
 
+def gen_state_dict_r18():
+    """Key -> shape table of the reference ResNet-18 volumetric model at a 32^3 grid (the train.py drop-in test's model)."""
+    import json
+    ref = RefNet(testing.make_config(num_layers=18, volume_size=32), device="cpu")
+    with open(os.path.join(HERE, "state_dict_r18.json"), "w") as f:
+        json.dump({k: list(v.shape) for k, v in ref.state_dict().items()}, f)
+
+
+def _checksum(tensors):
+    return float(sum(torch.as_tensor(t).double().abs().sum() for t in tensors))
+
+
+def gen_oracle_vs_reference():
+    """Reference outputs for tests/test_oracle_vs_reference.py: unprojection on random scenes, the coordinate volume and
+    projection of a ResNet-18 forward, and V2V / pose-ResNet-34 forwards (weights and inputs from torch.manual_seed(0)).
+    Large outputs are stored as a fixed seeded sample of SAMPLE draws (testing.golden_sample) plus per-channel means."""
+    from oracle import vol_oracle as O
+    from mvn.models import v2v as ref_v2v, pose_resnet as ref_pose_resnet
+    SAMPLE = 16384
+    out = {"sample_k": np.array([SAMPLE])}
+    for i, (B, V, C, h, w, n) in enumerate([(1, 2, 3, 9, 13, 5), (2, 8, 4, 12, 12, 6), (1, 9, 2, 8, 6, 4)]):
+        rng = np.random.RandomState(B * 100 + V)
+        heat = rng.randn(B, V, C, h, w).astype(np.float32)
+        cams = testing.make_cameras(V, image_size=48, radius=3000.0)
+        proj = np.stack([np.stack([O.projection_after_resize(c.K, c.R, c.t, (48, 48), (h, w)) for c in cams])] * B)
+        coord = np.stack([O.coord_volume(rng.randn(3) * 100 + [0, 0, 900], 2600.0, n) for _ in range(B)])
+        conf = rng.rand(B, V, C).astype(np.float32)
+        out["unp%d_inputs" % i] = np.array([testing.array_digest(a) for a in (heat, proj, coord, conf)])
+        for agg in ("sum", "max", "softmax", "conf"):
+            out["unp%d_out_%s" % (i, agg)] = ref_op.unproject_heatmaps(torch.from_numpy(heat), torch.from_numpy(proj),
+                                                                       torch.from_numpy(coord), agg, torch.from_numpy(conf)).numpy()
+
+    base = np.array([123.4, -56.7, 910.1])
+    net = RefNet(testing.make_config(num_layers=18, volume_size=32), device="cpu").eval()
+    images, batch = testing.make_batch(1, 2, image_size=64, seed=5, camera_cls=ref_multiview.Camera)
+    batch["keypoints_3d"][0][6, :3] = base
+    with torch.no_grad():
+        coords = net(images, None, batch)[5].numpy()[0]
+    # each coordinate depends on its own voxel index only, so three axes hold the whole volume bit for bit
+    axes = [coords[:, 0, 0, 0], coords[0, :, 0, 1], coords[0, 0, :, 2]]
+    full = np.stack(np.broadcast_arrays(axes[0][:, None, None], axes[1][None, :, None], axes[2][None, None, :]), -1)
+    assert np.array_equal(full, coords)
+    out["coord_base"] = base
+    out["coord_x"], out["coord_y"], out["coord_z"] = axes
+    cam = batch["cameras"][1][0]
+    c2 = ref_multiview.Camera(cam.R, cam.t, cam.K)
+    c2.update_after_resize((64, 64), (16, 16))
+    out["cam_K"], out["cam_R"], out["cam_t"] = cam.K, cam.R, cam.t
+    out["cam_projection_16"] = c2.projection.astype(np.float32)
+
+    torch.manual_seed(0)
+    v = ref_v2v.V2VModel(32, 17).eval()
+    for m in v.modules():
+        if isinstance(m, torch.nn.BatchNorm3d):
+            m.running_mean.normal_(0, 0.1)
+            m.running_var.uniform_(0.5, 1.5)
+    x = torch.randn(1, 32, 32, 32, 32)
+    with torch.no_grad():
+        want = v(x)
+    out["v2v_checksum"] = np.array([_checksum(v.state_dict().values()), _checksum([x])])
+    out["v2v_sample"] = testing.golden_sample(want.numpy(), SAMPLE)
+    out["v2v_channel_mean"] = want.double().mean((0, 2, 3, 4)).numpy()
+    out["v2v_absmax"] = np.array([float(want.abs().max())])
+    cfg = testing.AttrDict(num_layers=34, style="simple", num_joints=17, alg_confidences=False, vol_confidences=False,
+                           init_weights=False)
+    bb = ref_pose_resnet.get_pose_net(cfg, device="cpu").eval()
+    xi = torch.randn(2, 3, 64, 64)
+    with torch.no_grad():
+        hm, feats, _, _ = bb(xi)
+    out["backbone_checksum"] = np.array([_checksum(bb.state_dict().values()), _checksum([xi])])
+    out["backbone_heatmaps_sample"] = testing.golden_sample(hm.numpy(), SAMPLE)
+    out["backbone_heatmaps_absmax"] = np.array([float(hm.abs().max())])
+    out["backbone_features_sample"] = testing.golden_sample(feats.numpy(), SAMPLE)
+    out["backbone_features_channel_mean"] = feats.double().mean((0, 2, 3)).numpy()
+    out["backbone_features_absmax"] = np.array([float(feats.abs().max())])
+    np.savez_compressed(os.path.join(HERE, "oracle_vs_reference.npz"), **out)
+
+
+def gen_collate():
+    """Reference collate_fn / prepare_batch / normalize_image outputs for tests/test_pipeline_cpu.py, all compared for
+    exact equality there, so only their digests (testing.array_digest) are stored."""
+    from mvn.datasets import utils as ref_utils
+    from mvn.utils import img as ref_img
+    out = {}
+    for randomize in (False, True):
+        items = testing.dataset_items(3, 5, seed=9, camera_cls=ref_multiview.Camera)
+        np.random.seed(11)
+        want = ref_utils.make_collate_fn(randomize_n_views=randomize, min_n_views=2, max_n_views=4)(list(items))
+        key = "r%d_" % randomize
+        for name in ("images", "detections", "pred_keypoints_3d"):
+            out[key + name] = testing.array_digest(want[name])
+        # which item / view each collated camera is, [view][batch] -> (item, view)
+        where = {id(c): (b, v) for b, it in enumerate(items) for v, c in enumerate(it["cameras"])}
+        out[key + "camera_index"] = np.array([[where[id(c)] for c in row] for row in want["cameras"]])
+        out[key + "prepared"] = np.array([testing.array_digest(t.numpy()) for t in ref_utils.prepare_batch(want, "cpu", None)])
+    u8 = np.random.RandomState(1).randint(0, 256, size=(2, 2, 6, 7, 3)).astype(np.uint8)
+    ref_norm = np.stack([np.stack([ref_img.normalize_image(im) for im in row]) for row in u8])
+    out["u8_normalized"] = testing.array_digest(torch.stack([ref_img.image_batch_to_torch(x) for x in ref_norm]).numpy())
+    np.savez_compressed(os.path.join(HERE, "collate.npz"), **out)
+
+
 if __name__ == "__main__":
-    gen_state_dict_keys()
-    gen_unproject()
-    gen_softargmax()
-    gen_forward()
-    gen_algebraic()
+    fixtures = {"state_dict_r152": gen_state_dict_keys, "state_dict_r18": gen_state_dict_r18, "unproject": gen_unproject, "softargmax": gen_softargmax,
+                "forward_r50": gen_forward, "algebraic_r50": gen_algebraic, "oracle_vs_reference": gen_oracle_vs_reference,
+                "collate": gen_collate}
+    for name in sys.argv[2:] or fixtures:
+        fixtures[name]()
     for f in sorted(os.listdir(HERE)):
         print(f, os.path.getsize(os.path.join(HERE, f)))

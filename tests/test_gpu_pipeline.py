@@ -27,8 +27,7 @@ def test_images_to_device_native_equals_torch(dtype, shape):
 
 
 def test_pinned_collate_and_prepare_batch():
-    from test_pipeline_cpu import _items
-    items = _items(3, 4, size=16, dtype=np.float64, seed=2)
+    items = testing.dataset_items(3, 4, size=16, dtype=np.float64, seed=2)
     batch = pipeline.make_collate_fn(randomize_n_views=False, pinned=True)(items)
     assert torch.from_numpy(batch["images"]).is_pinned()
     native = pipeline.prepare_batch(batch, DEV, None)

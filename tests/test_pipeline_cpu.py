@@ -1,31 +1,14 @@
 """Host batch contract (lt_b200.pipeline): collate, normalisation table, prepare_batch (torch backend on CPU).
-Reference behaviours mirrored: mvn/datasets/utils.py:6-65, mvn/utils/img.py:96-110.  Where /root/reference is mounted
-(the authoring container) the same inputs also run through the reference functions."""
-import sys
+Reference behaviours mirrored: mvn/datasets/utils.py:6-65, mvn/utils/img.py:96-110.  What the reference functions return
+for the same inputs is stored as digests in tests/golden/collate.npz (tests/golden/make_golden.py)."""
+import os
 
 import numpy as np
 import pytest
 import torch
 
-from conftest import REFERENCE, has_reference
+from conftest import GOLDEN
 from lt_b200 import pipeline, testing
-
-
-def _items(n_items, n_views, size=8, dtype=np.float64, seed=0, camera_cls=None):
-    rng = np.random.RandomState(seed)
-    cams = testing.make_cameras(n_views, image_size=size)
-    if camera_cls is not None:
-        cams = [camera_cls(c.R, c.t, c.K) for c in cams]
-    items = []
-    for i in range(n_items):
-        if dtype == np.uint8:
-            imgs = [rng.randint(0, 256, size=(size, size + 2, 3)).astype(np.uint8) for _ in range(n_views)]
-        else:
-            imgs = [rng.randn(size, size + 2, 3).astype(dtype) for _ in range(n_views)]
-        items.append({"images": imgs, "detections": [rng.rand(5) for _ in range(n_views)], "cameras": list(cams),
-                      "keypoints_3d": rng.randn(17, 4).astype(np.float32), "indexes": i,
-                      "pred_keypoints_3d": rng.randn(17, 3)})
-    return items
 
 
 def test_normalization_table_is_normalize_image_rounded_once():
@@ -38,7 +21,7 @@ def test_normalization_table_is_normalize_image_rounded_once():
 
 
 def test_collate_layout_and_none_filtering(capsys):
-    items = _items(3, 4)
+    items = testing.dataset_items(3, 4)
     fn = pipeline.make_collate_fn(randomize_n_views=False)
     batch = fn([items[0], None, items[1], items[2]])
     assert batch["images"].shape == (3, 4, 8, 10, 3) and batch["images"].flags["C_CONTIGUOUS"]
@@ -54,7 +37,7 @@ def test_collate_layout_and_none_filtering(capsys):
 
 
 def test_collate_random_views_within_bounds():
-    items = _items(2, 6)
+    items = testing.dataset_items(2, 6)
     fn = pipeline.make_collate_fn(randomize_n_views=True, min_n_views=2, max_n_views=4)
     np.random.seed(3)
     seen = set()
@@ -68,7 +51,7 @@ def test_collate_random_views_within_bounds():
 
 @pytest.mark.parametrize("dtype", [np.float64, np.float32, np.uint8])
 def test_prepare_batch_torch_backend(dtype):
-    items = _items(2, 3, dtype=dtype, seed=4)
+    items = testing.dataset_items(2, 3, dtype=dtype, seed=4)
     batch = pipeline.make_collate_fn(randomize_n_views=False)(items)
     images, kp, valid, proj = pipeline.prepare_batch(batch, "cpu", None, backend="torch")
     assert images.shape == (2, 3, 3, 8, 10) and images.dtype == torch.float32
@@ -85,34 +68,25 @@ def test_prepare_batch_torch_backend(dtype):
 
 
 def test_native_backend_refuses_cpu_device():
-    batch = pipeline.make_collate_fn(randomize_n_views=False)(_items(1, 2))
+    batch = pipeline.make_collate_fn(randomize_n_views=False)(testing.dataset_items(1, 2))
     with pytest.raises(RuntimeError):
         pipeline.prepare_batch(batch, "cpu", None)          # default backend is the CUDA path: no silent CPU route
 
 
-@pytest.mark.skipif(not has_reference(), reason="reference checkout not mounted")
 @pytest.mark.parametrize("randomize", [False, True])
 def test_collate_and_prepare_batch_equal_reference(randomize):
-    sys.path.insert(0, REFERENCE)
-    from mvn.datasets import utils as ref_utils
-    from mvn.utils import img as ref_img
-    from mvn.utils.multiview import Camera as RefCamera
-    items = _items(3, 5, seed=9, camera_cls=RefCamera)
-    kw = dict(randomize_n_views=randomize, min_n_views=2, max_n_views=4)
+    ref = np.load(os.path.join(GOLDEN, "collate.npz"))
+    key = "r%d_" % randomize
+    items = testing.dataset_items(3, 5, seed=9)
     np.random.seed(11)
-    want = ref_utils.make_collate_fn(**kw)(list(items))
-    np.random.seed(11)
-    got = pipeline.make_collate_fn(**kw)(list(items))
-    assert np.array_equal(got["images"], want["images"]) and np.array_equal(got["detections"], want["detections"])
-    assert np.array_equal(got["pred_keypoints_3d"], want["pred_keypoints_3d"])
-    assert [[id(c) for c in row] for row in got["cameras"]] == [[id(c) for c in row] for row in want["cameras"]]
-    r = ref_utils.prepare_batch(want, "cpu", None)
+    got = pipeline.make_collate_fn(randomize_n_views=randomize, min_n_views=2, max_n_views=4)(list(items))
+    for name in ("images", "detections", "pred_keypoints_3d"):
+        assert testing.array_digest(got[name]) == ref[key + name], name
+    where = {id(c): (b, v) for b, it in enumerate(items) for v, c in enumerate(it["cameras"])}
+    assert np.array_equal([[where[id(c)] for c in row] for row in got["cameras"]], ref[key + "camera_index"])
     m = pipeline.prepare_batch(got, "cpu", None, backend="torch")
-    for a, b in zip(m, r):
-        assert a.dtype == b.dtype and torch.equal(a, b)
+    assert [testing.array_digest(t.numpy()) for t in m] == list(ref[key + "prepared"])
     # uint8 crops normalised through the table == normalize_image on the CPU, then the reference upload path
     u8 = np.random.RandomState(1).randint(0, 256, size=(2, 2, 6, 7, 3)).astype(np.uint8)
-    ref_norm = np.stack([np.stack([ref_img.normalize_image(im) for im in row]) for row in u8])
-    want_t = torch.stack([ref_img.image_batch_to_torch(x) for x in ref_norm])
     got_t = pipeline.images_to_device(u8, "cpu", normalize_u8=True, backend="torch")
-    assert torch.equal(got_t, want_t)
+    assert testing.array_digest(got_t.numpy()) == ref["u8_normalized"]

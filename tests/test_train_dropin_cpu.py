@@ -1,11 +1,13 @@
-"""Drop-in proof against the reference's own training script (only where /root/reference is mounted).
+"""Drop-in proof for the reference's training script, without the reference itself.
 
-Imports the UNMODIFIED `/root/reference/train.py` (its missing optional dependencies -- tensorboardX, matplotlib, skimage,
-easydict, h5py -- stubbed), calls `lt_b200.install()`, and then walks the exact statements of `train.py` that touch the
-model: construction from the experiment yaml (train.py:400-404), strict `load_state_dict` of a checkpoint with DDP's
-`module.` prefixes (:406-413), the three optimizer parameter groups (:430-437), `DistributedDataParallel` wrapping
-(:452-453, gloo, world_size 2) and one forward/backward/step of the loop body (:189-243) on the CPU (`backend="torch"`).
+`lt_b200.install()` rebinds the names `train.py` imports (tested on a stand-in `mvn` package); then the statements of
+`train.py` that touch the model run against lt_b200's class as `train.py` would call it: construction from the experiment
+config with the backend chosen by LT_B200_BACKEND (train.py:400-404), strict `load_state_dict` of a checkpoint with DDP's
+`module.` prefixes and the reference's key set (:406-413, key/shape table in tests/golden/state_dict_r18.json), the three
+optimizer parameter groups (:430-437), `DistributedDataParallel` wrapping (:452-453, gloo, world_size 2) and one
+forward/backward/step of the loop body (:189-243) on the CPU.
 """
+import json
 import os
 import socket
 import sys
@@ -16,132 +18,101 @@ import pytest
 import torch
 import torch.multiprocessing as mp
 
-from conftest import REFERENCE, has_reference
-
-pytestmark = pytest.mark.skipif(not has_reference(), reason="reference checkout not mounted")
+from conftest import GOLDEN
 
 
-def _stub_missing_modules():
-    """Minimal stand-ins for the reference's optional third-party imports that this image lacks."""
-    def mod(name, **attrs):
-        if name in sys.modules:
-            return sys.modules[name]
-        m = types.ModuleType(name)
-        m.__dict__.update(attrs)
-        sys.modules[name] = m
-        return m
-
-    class _Writer:
-        def __init__(self, *a, **k): pass
-        def add_scalar(self, *a, **k): pass
-        def add_image(self, *a, **k): pass
-        def add_text(self, *a, **k): pass
-        def close(self): pass
-
-    class _EasyDict(dict):
-        def __init__(self, d=None, **kw):
-            super().__init__()
-            for k, v in dict(d or {}, **kw).items():
-                setattr(self, k, v)
-
-        def __setattr__(self, k, v):
-            v = _EasyDict(v) if isinstance(v, dict) and not isinstance(v, _EasyDict) else v
-            super().__setitem__(k, v)
-            super().__setattr__(k, v)
-        __setitem__ = __setattr__
-
-    try:
-        import tensorboardX  # noqa: F401
-    except ImportError:
-        mod("tensorboardX", SummaryWriter=_Writer)
-    try:
-        import easydict  # noqa: F401
-    except ImportError:
-        mod("easydict", EasyDict=_EasyDict)
-    try:
-        import matplotlib  # noqa: F401
-    except ImportError:
-        mpl = mod("matplotlib", use=lambda *a, **k: None)
-        mpl.pylab = mod("matplotlib.pylab")
-        mpl.pyplot = mod("matplotlib.pyplot")
-        tk = mod("mpl_toolkits")
-        tk.mplot3d = mod("mpl_toolkits.mplot3d", axes3d=None, Axes3D=None)
-    try:
-        import skimage  # noqa: F401
-    except ImportError:
-        sk = mod("skimage")
-        sk.transform = mod("skimage.transform")
-    try:
-        import h5py  # noqa: F401
-    except ImportError:
-        mod("h5py")
-
-
-def _import_reference_train():
-    _stub_missing_modules()
-    if REFERENCE not in sys.path:
-        sys.path.insert(0, REFERENCE)
-    import lt_b200
-    import mvn  # noqa: F401
-    lt_b200.install()               # BEFORE train.py binds the class names (`from mvn.models.triangulation import ...`)
-    import importlib
-    train = importlib.import_module("train")
-    return lt_b200, train
-
-
-def _tiny_config(train):
-    """The reference's own yaml (experiments/human36m/train/human36m_vol_softmax.yaml) shrunk for a CPU test."""
-    from mvn.utils import cfg
-    config = cfg.load_config(os.path.join(REFERENCE, "experiments/human36m/train/human36m_vol_softmax.yaml"))
-    config.model.init_weights = False
-    config.model.backbone.init_weights = False
-    config.model.backbone.name = "resnet18"
-    config.model.backbone.num_layers = 18
-    config.model.volume_size = 32
+def _tiny_config():
+    """experiments/human36m/train/human36m_vol_softmax.yaml shrunk for a CPU test: ResNet-18 backbone, 32^3 grid, no
+    pretrained weights.  The yaml differs from testing.make_config only in use_gt_pelvis; `opt` holds its learning rates."""
+    from lt_b200 import testing
+    config = testing.make_config(num_layers=18, volume_size=32, use_gt_pelvis=False)
+    config.opt = testing.AttrDict(lr=1e-4, process_features_lr=1e-3, volume_net_lr=1e-3)
     return config
 
 
-def test_install_patches_the_names_train_py_binds():
-    lt_b200, train = _import_reference_train()
-    assert train.VolumetricTriangulationNet is lt_b200.VolumetricTriangulationNet
-    assert train.AlgebraicTriangulationNet is lt_b200.AlgebraicTriangulationNet
-    from mvn.utils import op as ref_op
+def _build_model(config, device="cpu"):
+    """train.py:400-404: the class is called with (config, device) only; the backend comes from the environment."""
+    import lt_b200
+    os.environ["LT_B200_BACKEND"] = "torch"
+    try:
+        return lt_b200.VolumetricTriangulationNet(config, device=device).to(device)
+    finally:
+        os.environ.pop("LT_B200_BACKEND")
+
+
+def _keypoints_mae(pred, gt, validity):
+    """The MAE criterion train.py selects (opt.criterion: MAE): masked mean absolute error over joints and coordinates."""
+    return torch.sum(torch.abs(gt - pred) * validity) / (pred.shape[-1] * max(1, float(validity.sum())))
+
+
+@pytest.fixture
+def stand_in_mvn():
+    """A package shaped like the reference's `mvn`, holding placeholders where install() must put lt_b200's objects."""
+    name = "mvn_stand_in"
+    mods = {}
+    for sub in ("", ".models", ".models.triangulation", ".utils", ".utils.op"):
+        mods[name + sub] = types.ModuleType(name + sub)
+    tri, op = mods[name + ".models.triangulation"], mods[name + ".utils.op"]
+    for attr in ("VolumetricTriangulationNet", "AlgebraicTriangulationNet", "RANSACTriangulationNet"):
+        setattr(tri, attr, type(attr, (), {}))
+    for attr in ("integrate_tensor_2d", "unproject_heatmaps", "integrate_tensor_3d_with_coordinates"):
+        setattr(op, attr, lambda *a, **k: None)
+    mods[name].models, mods[name].utils = mods[name + ".models"], mods[name + ".utils"]
+    mods[name + ".models"].triangulation, mods[name + ".utils"].op = tri, op
+    sys.modules.update(mods)
+    try:
+        yield mods[name]
+    finally:
+        for key in mods:
+            sys.modules.pop(key, None)
+
+
+def test_install_patches_the_names_train_py_binds(stand_in_mvn):
+    import lt_b200
+    ransac = stand_in_mvn.models.triangulation.RANSACTriangulationNet
+    assert lt_b200.install(stand_in_mvn) is stand_in_mvn
+    tri, ref_op = stand_in_mvn.models.triangulation, stand_in_mvn.utils.op
+    assert tri.VolumetricTriangulationNet is lt_b200.VolumetricTriangulationNet
+    assert tri.AlgebraicTriangulationNet is lt_b200.AlgebraicTriangulationNet
+    assert tri.RANSACTriangulationNet is ransac                       # not replaced: no native implementation
+    assert ref_op.integrate_tensor_2d is lt_b200.op.integrate_tensor_2d
     assert ref_op.unproject_heatmaps is lt_b200.op.unproject_heatmaps
     assert ref_op.integrate_tensor_3d_with_coordinates is lt_b200.op.integrate_tensor_3d_with_coordinates
+    # what train.py does at import time, after install()
+    scope = {}
+    exec("from mvn_stand_in.models.triangulation import VolumetricTriangulationNet, AlgebraicTriangulationNet", scope)
+    assert scope["VolumetricTriangulationNet"] is lt_b200.VolumetricTriangulationNet
+    assert scope["AlgebraicTriangulationNet"] is lt_b200.AlgebraicTriangulationNet
 
 
 def test_train_py_model_setup_statements():
     """train.py:400-413 (construct + strict load of a DDP-prefixed checkpoint) and :430-437 (optimizer parameter groups)."""
-    lt_b200, train = _import_reference_train()
-    config = _tiny_config(train)
-    device = torch.device("cpu")
-    os.environ["LT_B200_BACKEND"] = "torch"
-    try:
-        model = {"ransac": train.RANSACTriangulationNet, "alg": train.AlgebraicTriangulationNet,
-                 "vol": train.VolumetricTriangulationNet}[config.model.name](config, device=device).to(device)      # train.py:400-404
-    finally:
-        os.environ.pop("LT_B200_BACKEND")
-    assert isinstance(model, lt_b200.VolumetricTriangulationNet)
-    # the reference class itself gives the key set a released checkpoint would carry
-    import importlib
-    ref_tri = importlib.import_module("mvn.models.triangulation")
-    importlib.reload(ref_tri)                      # un-patched class object
-    ref_model = ref_tri.VolumetricTriangulationNet(_tiny_config(train), device="cpu")
-    lt_b200.install()
-    state_dict = {"module." + k: v for k, v in ref_model.state_dict().items()}          # as saved under DDP (train.py:465-469)
+    import lt_b200
+    config = _tiny_config()
+    model = _build_model(config)
+    assert isinstance(model, lt_b200.VolumetricTriangulationNet) and model.backend == "torch"
+    # a checkpoint with the reference model's key set, as saved under DDP (train.py:465-469)
+    shapes = json.load(open(os.path.join(GOLDEN, "state_dict_r18.json")))
+    g = torch.Generator().manual_seed(0)
+    saved = {k: torch.randn(s, generator=g) if s else torch.randint(0, 100, (), generator=g) for k, s in shapes.items()}
+    state_dict = {"module." + k: v for k, v in saved.items()}
     for key in list(state_dict.keys()):                                                  # train.py:408-410
         new_key = key.replace("module.", "")
         state_dict[new_key] = state_dict.pop(key)
     model.load_state_dict(state_dict, strict=True)                                       # train.py:412
-    for k, v in ref_model.state_dict().items():
-        assert torch.equal(model.state_dict()[k], v)
+    have = model.state_dict()
+    assert set(have) == set(saved)
+    for k, v in saved.items():
+        assert torch.equal(have[k], v.to(have[k].dtype)), k
     opt = torch.optim.Adam(                                                              # train.py:430-437
         [{'params': model.backbone.parameters()},
          {'params': model.process_features.parameters(), 'lr': config.opt.process_features_lr if hasattr(config.opt, "process_features_lr") else config.opt.lr},
          {'params': model.volume_net.parameters(), 'lr': config.opt.volume_net_lr if hasattr(config.opt, "volume_net_lr") else config.opt.lr}],
         lr=config.opt.lr)
-    n_opt = sum(p.numel() for g in opt.param_groups for p in g["params"])
-    assert n_opt == sum(p.numel() for p in model.parameters())
+    assert [g["lr"] for g in opt.param_groups] == [1e-4, 1e-3, 1e-3]
+    in_groups = [p for g in opt.param_groups for p in g["params"]]
+    assert len({id(p) for p in in_groups}) == len(in_groups)                             # no parameter in two groups
+    assert {id(p) for p in in_groups} == {id(p) for p in model.parameters()}             # and none left out
     assert not any(p.requires_grad for p in model.backbone.final_layer.parameters())     # frozen head, triangulation.py:235-236
 
 
@@ -152,18 +123,13 @@ def _free_port():
 def _ddp_worker(rank, world, port, ret):
     import torch.distributed as dist
     from torch.nn.parallel import DistributedDataParallel
-    sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__))))
     os.environ["MASTER_ADDR"], os.environ["MASTER_PORT"] = "127.0.0.1", str(port)
     dist.init_process_group("gloo", rank=rank, world_size=world)
     try:
-        lt_b200, train = _import_reference_train()
         from lt_b200 import testing
-        config = _tiny_config(train)
         torch.manual_seed(0)
-        os.environ["LT_B200_BACKEND"] = "torch"
-        model = train.VolumetricTriangulationNet(config, device="cpu").to("cpu")
+        model = _build_model(_tiny_config())
         model = DistributedDataParallel(model)                                           # train.py:452-453 (device_ids=None on CPU)
-        criterion = train.KeypointsMAELoss()
         opt = torch.optim.Adam(filter(lambda p: p.requires_grad, model.parameters()), lr=1e-4)
         images, batch = testing.make_batch(2, 2, image_size=64, seed=10 + rank)   # 2 samples: train-mode BN at the 1^3 V2V level
         model.train()
@@ -171,7 +137,7 @@ def _ddp_worker(rank, world, port, ret):
             model(images, None, batch)                                                   # train.py:189-191
         gt = torch.from_numpy(np.stack(batch["keypoints_3d"])[:, :, :3]).float()
         validity = torch.ones(2, 17, 1)
-        loss = criterion(keypoints_3d_pred * 0.1, gt * 0.1, validity)                    # train.py:219-221 (scale_keypoints_3d)
+        loss = _keypoints_mae(keypoints_3d_pred * 0.1, gt * 0.1, validity)               # train.py:219-221 (scale_keypoints_3d)
         opt.zero_grad()
         loss.backward()                                                                  # train.py:236
         g = model.module.process_features[0].weight.grad.clone()
@@ -179,7 +145,8 @@ def _ddp_worker(rank, world, port, ret):
         # DDP averaged the gradient: identical on both ranks although the inputs differ
         gathered = [torch.zeros_like(g) for _ in range(world)]
         dist.all_gather(gathered, g)
-        ret[rank] = (float(loss), bool(torch.equal(gathered[0], gathered[1])), tuple(keypoints_3d_pred.shape))
+        ret[rank] = (float(loss), bool(torch.equal(gathered[0], gathered[1])), tuple(keypoints_3d_pred.shape),
+                     float(g.abs().sum()))
     finally:
         dist.destroy_process_group()
 
@@ -190,5 +157,5 @@ def test_ddp_wrap_and_one_training_step_gloo():
     ret = mp.get_context("spawn").Manager().dict()
     mp.spawn(_ddp_worker, args=(world, _free_port(), ret), nprocs=world, join=True)
     assert len(ret) == world
-    for rank, (loss, same_grad, shape) in ret.items():
-        assert np.isfinite(loss) and same_grad and shape == (2, 17, 3)
+    for rank, (loss, same_grad, shape, grad_mass) in ret.items():
+        assert np.isfinite(loss) and same_grad and shape == (2, 17, 3) and grad_mass > 0
